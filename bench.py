@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path on the host cores
+  python bench.py ... --dump-outputs DIR                    # also saves the last timed step's outputs, to compare builds
 
 A "step" is one pass of the hot path (joint forward -> alpha/beta -> gradients to enc_acts, pred_acts,
 W, b) over one synthetic batch of the BASELINE C3 shape (B=32,T=512,U=128,V=1024,H=640 per GPU, bf16
@@ -27,6 +28,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the source tree (it may be read-only)
 
 WORKLOADS = {
     "c3": dict(B=32, T=512, U=128, V=1024, H=640, precision="bf16", dtype="bf16"),
@@ -37,6 +39,28 @@ WORKLOADS = {
     "c5": dict(B=64, T=1600, U=200, V=4096, H=640, precision="bf16", dtype="bf16", ragged=True),
 }
 METRIC = "rnnt_loss_grad_utterances_per_sec"
+# what one step hands its caller, in the order step() returns it
+OUTPUT_NAMES = ("loss", "costs", "d_enc", "d_pred", "dW", "db")
+DUMP_BYTES = 64 * 10 ** 6              # all files of --dump-outputs together
+
+
+def dump_sample(named):
+    """{name: float32 numpy array} of the device tensors in `named`: whole when together they fit DUMP_BYTES; otherwise the
+    larger ones are cut to a fixed, seeded sample of their flattened elements (in index order) so that the total fits.
+    The sample depends on the shapes only, so two runs with the same arguments dump the same elements."""
+    import numpy as np
+    import torch
+    sizes = {n: t.numel() for n, t in named.items()}
+    left, out = (DUMP_BYTES - 1024 * len(named)) // 4, {}            # 1 KiB per file for the .npy header
+    for i, n in enumerate(sorted(sizes, key=sizes.get)):
+        keep = min(sizes[n], left // (len(sizes) - i))
+        left -= keep
+        t = named[n].detach().float()
+        if keep < sizes[n]:
+            idx = np.sort(np.random.default_rng(0).choice(sizes[n], keep, replace=False, shuffle=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        out[n] = t.cpu().numpy()
+    return out
 
 
 def peaks():
@@ -260,7 +284,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-op-path", action="store_true")
     ap.add_argument("--cpu-budget", type=float, default=20.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (%s) to DIR/<name>.npy as float32, at most %d MB in "
+                         "all: beyond that the larger arrays become a fixed, seeded sample of their flattened elements; "
+                         "rank 0 only" % (", ".join(OUTPUT_NAMES), DUMP_BYTES // 10 ** 6))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -314,7 +346,7 @@ def main():
         loss_sum = costs.sum()
         (loss_sum / mode["gB"]).backward()                           # run_rnnt.py:278
         ls, dW, db = D.allreduce_loss_and_weight_grads(loss_sum.detach(), params[0].grad, params[1].grad)
-        return ls / mode["gB"], enc.grad, pred.grad, dW, db
+        return ls / mode["gB"], costs.detach(), enc.grad, pred.grad, dW, db          # OUTPUT_NAMES
 
     cur = {"d": d}
 
@@ -346,15 +378,20 @@ def main():
         out = step(dd["enc"], dd["pred"], dd["labels"], dd["il"], dd["ll"])
         return out[0].item()                                          # D2H read of the step's loss
 
-    def timed(fn, steps):
+    def timed(fn, steps, keep=None):
+        """Milliseconds of `steps` calls of fn.  keep: a dict that receives what the LAST call returned; every other call's
+        result is dropped at once, as a caller's would be, so that no step holds its predecessor's outputs in memory."""
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
-        for a, b in ev:
+        for i, (a, b) in enumerate(ev):
             flush.zero_()                                             # L2 flush, outside the event pair
             a.record()
-            fn()
+            if keep is None or i + 1 < steps:
+                fn()
+            else:
+                keep["out"] = fn()
             b.record()
         torch.cuda.synchronize()
         if world > 1:
@@ -371,8 +408,10 @@ def main():
     if sampler:
         sampler.start()
     l0 = _lib.launch_count()
-    ms = timed(resident_step, args.steps)
+    last = {} if args.dump_outputs and rank == 0 else None
+    ms = timed(resident_step, args.steps, keep=last)
     launches = _lib.launch_count() - l0
+    dumped = dump_sample(dict(zip(OUTPUT_NAMES, last.pop("out")))) if last is not None else None
     for _ in range(2):
         e2e_step()
     ms_e2e = timed(e2e_step, args.steps)
@@ -465,6 +504,11 @@ def main():
             out["op_path"] = op_path_block(pk)
         if world == 1 and not args.no_cpu_baseline:
             out["cpu_baseline"] = cpu_baseline(cfg, args.cpu_budget)
+        if dumped:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for n, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, n + ".npy"), a)
         sys.stdout.flush()
         os.write(real_stdout, (json.dumps(out) + "\n").encode())
     if world > 1:

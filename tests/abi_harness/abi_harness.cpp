@@ -1,24 +1,44 @@
-// Link-level check of the drop-in boundary: this translation unit includes the REFERENCE's own header
-// (warp-transducer/include/rnnt.h, found through -I at build time -- it is not copied into this repo) and is linked
-// against librnnt_b200.so.  It is what a binding such as tensorflow_binding/src/warprnnt_op.cc:105-141 or
-// pytorch_binding/src/binding.cpp:84-154 does with the library: get_workspace_size -> device workspace ->
-// compute_rnnt_loss(RNNT_GPU, device labels/lengths, HOST costs) -> status string.
+// Link-level check of the drop-in boundary: this translation unit uses the warp-transducer API (rnnt.h) through this
+// project's drop-in header include/rnnt_b200.h and is linked against librnnt_b200.so.  It is what a binding such as
+// tensorflow_binding/src/warprnnt_op.cc:105-141 or pytorch_binding/src/binding.cpp:84-154 does with the library:
+// get_workspace_size -> device workspace -> compute_rnnt_loss(RNNT_GPU, device labels/lengths, HOST costs) -> status
+// string.  Built with -DRNNT_REFERENCE_HEADER it includes the reference's own rnnt.h instead (found through -I, never
+// copied into this repo): tests/golden/make_golden.py does so to record the reference header's layout, which
+// tests/test_abi.py holds this header's layout to.
 // Data: the reference's own known-answer test (tests/test_cpu.cpp:12-71 / test_gpu.cu small_test): B=1 T=2 U=3 V=5,
 // expected cost 4.495666 and the logits gradient of pytorch_binding/test/test.py:62-74.
-// Modes:  abi_harness link   -> resolves every symbol and checks the host-only entry points (no GPU needed)
+// Modes:  abi_harness layout -> prints the rnntOptions layout and the enum values as one JSON line
+//         abi_harness link   -> resolves every symbol and checks the host-only entry points (no GPU needed)
 //         abi_harness run    -> runs the KAT on cuda:0
+#ifdef RNNT_REFERENCE_HEADER
 #include <rnnt.h>
+#else
+#include <rnnt_b200.h>
+#endif
 
 #include <cuda_runtime.h>
 
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <vector>
 
 static int fail(const char* what) { std::fprintf(stderr, "abi_harness: FAILED: %s\n", what); return 1; }
 
+static void print_layout() {
+    std::printf("{\"sizeof_rnntOptions\": %zu, \"offsets\": {\"loc\": %zu, \"num_threads\": %zu, \"stream\": %zu, "
+                "\"blank_label\": %zu, \"maxT\": %zu, \"maxU\": %zu, \"batch_first\": %zu}, "
+                "\"status\": [%d, %d, %d, %d, %d], \"location\": [%d, %d]}\n",
+                sizeof(rnntOptions), offsetof(rnntOptions, loc), offsetof(rnntOptions, num_threads),
+                offsetof(rnntOptions, stream), offsetof(rnntOptions, blank_label), offsetof(rnntOptions, maxT),
+                offsetof(rnntOptions, maxU), offsetof(rnntOptions, batch_first),
+                (int)RNNT_STATUS_SUCCESS, (int)RNNT_STATUS_MEMOPS_FAILED, (int)RNNT_STATUS_INVALID_VALUE,
+                (int)RNNT_STATUS_EXECUTION_FAILED, (int)RNNT_STATUS_UNKNOWN_ERROR, (int)RNNT_CPU, (int)RNNT_GPU);
+}
+
 int main(int argc, char** argv) {
+    if (argc > 1 && !std::strcmp(argv[1], "layout")) { print_layout(); return 0; }
     const bool run = argc > 1 && !std::strcmp(argv[1], "run");
     if (get_warprnnt_version() != 1) return fail("get_warprnnt_version");
     if (std::strcmp(rnntGetStatusString(RNNT_STATUS_SUCCESS), "no error")) return fail("status string");

@@ -16,12 +16,18 @@ Sources of truth, in order:
        reference): model.py:158-166 restated in torch fp64, chained by autograd through
        torch log_softmax (utils/loss.py:30) into the reference library's fp64 entry point
        (compute_rnnt_loss_fp64, rnnt.h:115-124).
+  4. The reference header's ABI (reference_abi.json): the functions rnnt.h declares, the
+       rnntOptions layout and enum values that tests/abi_harness reports when it is compiled
+       against rnnt.h, and the reference library's version and status strings.
 """
 import ast
 import ctypes as C
+import json
 import os
 import re
+import subprocess
 import sys
+import tempfile
 
 import numpy as np
 import torch
@@ -162,6 +168,90 @@ def joint_case(rng, B, T, U, V, H, blank=0, ragged=False):
                 dW=t[2].grad.numpy(), db=t[3].grad.numpy())
 
 
+def ref_cpu_case(acts, labels, il, ll, blank):
+    """Log-probs of `acts` through the reference's fp32 CPU path: what tests/test_oracle.py holds the oracle to."""
+    lp = oracle.log_softmax(acts)
+    costs, grads = oracle.ref_cpu_cost_and_grad(lp, labels, il, ll, blank=blank, num_threads=1)
+    return dict(log_probs=lp, labels=labels, input_lengths=il, label_lengths=ll, blank=np.int32(blank), costs=costs,
+                grads=grads)
+
+
+def ref_cpu_random_case():
+    """Fresh random input, ragged down to a single frame and an empty transcript, plus the reference's GPU workspace size."""
+    rng = np.random.default_rng(99)
+    B, T, U, V = 4, 13, 6, 9
+    acts = rng.standard_normal((B, T, U, V)).astype(np.float32)
+    labels = rng.integers(1, V, (B, U - 1)).astype(np.int32)
+    k = ref_cpu_case(acts, labels, np.array([13, 7, 1, 10], np.int32), np.array([5, 2, 0, 4], np.int32), 0)
+    sz = C.c_size_t(0)
+    assert oracle.ref().get_workspace_size(T, U, B, True, C.byref(sz), 4) == 0
+    k["gpu_workspace_bytes"] = np.int64(sz.value)
+    return k
+
+
+# (B, T, U, V, seed, logit scale): the 40 examples hypothesis draws (derandomized) from B in [1,4], T in [1,12],
+# U in [1,7], V in [2,11], scale in {0.3, 1, 6} -- boundary shapes first, then shrinks of larger ones
+PROPERTY_CASES = [
+    (1, 1, 1, 2, 0, 0.3), (2, 1, 1, 2, 0, 0.3), (2, 8, 7, 2, 9197, 6.0), (1, 12, 1, 2, 0, 0.3), (1, 12, 6, 5, 104017, 1.0),
+    (4, 9, 5, 11, 1764902504, 6.0), (4, 2, 4, 5, 13649451, 1.0), (3, 10, 5, 7, 4466, 1.0), (3, 1, 1, 3, 23782899, 6.0),
+    (4, 10, 6, 8, 22369, 6.0), (4, 9, 7, 2, 500, 0.3), (4, 9, 7, 7, 500, 0.3), (4, 9, 1, 7, 500, 0.3), (4, 7, 1, 7, 500, 0.3),
+    (4, 7, 1, 4, 500, 0.3), (4, 7, 1, 2, 500, 0.3), (4, 7, 1, 2, 2, 0.3), (4, 1, 2, 10, 532, 6.0), (4, 1, 1, 10, 532, 6.0),
+    (4, 1, 1, 2, 532, 6.0), (4, 1, 1, 2, 2, 6.0), (4, 1, 2, 2, 2, 6.0), (4, 2, 2, 2, 2, 6.0), (2, 2, 2, 2, 2, 6.0),
+    (2, 9, 3, 2, 99999999, 1.0), (1, 9, 3, 2, 99999999, 1.0), (1, 9, 3, 2, 9, 1.0), (1, 2, 3, 2, 9, 1.0), (1, 2, 1, 2, 9, 1.0),
+    (1, 1, 1, 2, 9, 1.0), (1, 1, 1, 2, 1, 1.0), (1, 4, 3, 2, 1561, 6.0), (1, 1, 3, 2, 1561, 6.0), (1, 1, 3, 2, 2, 6.0),
+    (1, 1, 3, 2, 1, 6.0), (1, 1, 1, 2, 1, 6.0), (1, 1, 1, 2, 2, 6.0), (4, 8, 1, 6, 3199819, 0.3), (4, 8, 1, 2, 3199819, 0.3),
+    (4, 2, 1, 2, 3199819, 0.3)]
+
+
+def ref_cpu_property_case(B, T, U, V, seed, scale):
+    """Random shape, ragged lengths, random blank position and logit scale."""
+    rng = np.random.default_rng(seed)
+    acts = (scale * rng.standard_normal((B, T, U, V))).astype(np.float32)
+    blank = int(rng.integers(0, V))
+    cand = np.array([v for v in range(V) if v != blank])
+    labels = (rng.choice(cand, size=(B, U - 1)).astype(np.int32) if U > 1 else np.zeros((B, 0), np.int32))
+    il = rng.integers(1, T + 1, B).astype(np.int32)
+    ll = rng.integers(0, U, B).astype(np.int32)
+    il[0], ll[0] = T, U - 1                       # the reference sizes its slabs by maxT / maxU
+    return ref_cpu_case(acts, labels, il, ll, blank)
+
+
+def joint_property_cases():
+    """Ten small random joint cases beyond the named fixtures (random blank, half of them ragged)."""
+    rng = np.random.default_rng(20260924)
+    out = []
+    for _ in range(10):
+        B, T, U = int(rng.integers(1, 4)), int(rng.integers(1, 9)), int(rng.integers(1, 6))
+        V, H = int(rng.integers(2, 9)), int(rng.integers(1, 7))
+        out.append(joint_case(rng, B, T, U, V, H, blank=int(rng.integers(0, V)), ragged=bool(rng.integers(0, 2))))
+    return out
+
+
+def save_cases(path, cases):
+    """Several cases of different shapes in one .npz: case i's arrays under "c<ii>_<name>"."""
+    np.savez_compressed(path, **{"c%02d_%s" % (i, n): a for i, k in enumerate(cases) for n, a in k.items()})
+
+
+def reference_abi():
+    """tests/abi_harness compiled against the reference's rnnt.h (and linked against this library, which it needs to
+    link) reports the header's rnntOptions layout and enum values; the version and status strings are the reference
+    library's own."""
+    hdr = open(os.path.join(REF, "include", "rnnt.h")).read()
+    hdr = re.sub(r"/\*.*?\*/", "", hdr, flags=re.S)
+    funcs = sorted(set(re.findall(r"^\s*(?:rnntStatus_t|int|const char\*)\s+(\w+)\s*\(", hdr, flags=re.M)))
+    pkg = os.path.join(ROOT, "rnnt_speech_recognition_b200")
+    with tempfile.TemporaryDirectory() as tmp:
+        exe = os.path.join(tmp, "abi_harness")
+        subprocess.run(["g++", "-O1", "-std=c++14", "-DRNNT_REFERENCE_HEADER", "-I" + os.path.join(REF, "include"),
+                        "-I/usr/local/cuda/include", os.path.join(ROOT, "tests", "abi_harness", "abi_harness.cpp"),
+                        "-L" + pkg, "-l:librnnt_b200.so", "-L/usr/local/cuda/lib64", "-lcudart", "-Wl,-rpath," + pkg,
+                        "-Wl,-rpath,/usr/local/cuda/lib64", "-o", exe], check=True)
+        layout = json.loads(subprocess.run([exe, "layout"], check=True, capture_output=True, text=True).stdout)
+    R = oracle.ref()
+    return {"header_functions": funcs, "layout": layout, "version": R.get_warprnnt_version(),
+            "status_strings": [R.rnntGetStatusString(i).decode() for i in range(6)]}
+
+
 def main():
     assert oracle.have_ref(), "needs oracle/_ref/libwarprnnt.so (make -C oracle)"
     kats = parse_pytorch_kats()
@@ -199,7 +289,13 @@ def main():
     }
     for k, v in jc.items():
         np.savez_compressed(os.path.join(HERE, "joint_%s.npz" % k), **v)
-    print("wrote", len(cases) + len(jc) + 2, "fixtures to", HERE)
+    np.savez_compressed(os.path.join(HERE, "refcpu_random_B4_T13_U6_V9.npz"), **ref_cpu_random_case())
+    save_cases(os.path.join(HERE, "refcpu_property_cases.npz"), [ref_cpu_property_case(*c) for c in PROPERTY_CASES])
+    save_cases(os.path.join(HERE, "jointchain_property_cases.npz"), joint_property_cases())
+    with open(os.path.join(HERE, "reference_abi.json"), "w") as f:
+        json.dump(reference_abi(), f, indent=1)
+        f.write("\n")
+    print("wrote", len(cases) + len(jc) + 6, "fixtures to", HERE)
 
 
 if __name__ == "__main__":

@@ -146,14 +146,12 @@ def test_forward_backward_likelihood_agree(L):
 
 
 def test_abi_harness_kat():
-    """The C++ harness built against the reference's own rnnt.h (tests/abi_harness) runs the reference's small_test
-    KAT (tests/test_cpu.cpp:12-71) through compute_rnnt_loss on the GPU: cost 4.495666 and the first gradient row."""
-    import os
+    """The C++ harness that uses the warp-transducer API through include/rnnt_b200.h (tests/abi_harness) runs the
+    reference's small_test KAT (tests/test_cpu.cpp:12-71) through compute_rnnt_loss on the GPU: cost 4.495666 and the
+    first gradient row."""
     import subprocess
-    from conftest import ROOT
-    exe = os.path.join(ROOT, "tests", "abi_harness", "_build", "abi_harness")
-    if not os.path.exists(exe):
-        pytest.skip("harness not prebuilt (needs /root/reference at build time)")
+    import __graft_entry__ as ge
+    exe = ge.build_abi_harness()
     r = subprocess.run([exe, "run"], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0, r.stdout + r.stderr
     assert "run ok" in r.stdout

@@ -1,10 +1,16 @@
-"""Pin the oracle (oracle/rnnt_oracle.c) against the reference's own known-answer tests, the
-golden fixtures generated from the reference library (tests/golden/make_golden.py) and, when it
-is present in this container, the unmodified reference library itself (oracle/_ref)."""
+"""Pin the oracle (oracle/rnnt_oracle.c) against the reference's own known-answer tests and the
+golden fixtures generated from the unmodified reference library (tests/golden/make_golden.py)."""
 import numpy as np
 import pytest
 
 from conftest import assert_close, fp32_tol, golden_names, load
+
+
+def load_cases(name):
+    """The cases of a multi-case fixture (tests/golden/make_golden.py: save_cases), in order."""
+    k = load(name)
+    n = len({key.split("_", 1)[0] for key in k})
+    return [{key.split("_", 1)[1]: v for key, v in k.items() if key.startswith("c%02d_" % i)} for i in range(n)]
 
 
 def softmax_chain(lp_grads, log_probs):
@@ -108,24 +114,15 @@ def test_numeric_gradient(oracle):
 
 
 def test_against_live_reference(oracle):
-    """When the unmodified reference library is available (this container, or shipped to the GPU
-    box in oracle/_ref) the restatement must agree with it on fresh random input."""
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref/libwarprnnt.so not available")
-    rng = np.random.default_rng(99)
-    B, T, U, V = 4, 13, 6, 9
-    acts = rng.standard_normal((B, T, U, V)).astype(np.float32)
-    labels = rng.integers(1, V, (B, U - 1)).astype(np.int32)
-    il = np.array([13, 7, 1, 10], np.int32)
-    ll = np.array([5, 2, 0, 4], np.int32)
-    lp = oracle.log_softmax(acts)
-    c, g = oracle.rnnt_cost_and_grad(lp, labels, il, ll)
-    cr, gr = oracle.ref_cpu_cost_and_grad(lp, labels, il, ll, num_threads=2)
-    assert np.allclose(c, cr, rtol=1e-6) and np.allclose(g, gr, rtol=1e-5, atol=1e-7)
-    rc, sz = oracle.get_workspace_size(T, U, B, True)
-    import ctypes as C
-    s = C.c_size_t(0)
-    assert oracle.ref().get_workspace_size(T, U, B, True, C.byref(s), 4) == rc == 0 and s.value == sz
+    """The restatement agrees with the unmodified reference library's fp32 CPU path (its costs and log-prob gradients,
+    recorded in tests/golden/refcpu_random_B4_T13_U6_V9.npz) on random input ragged down to a single frame and an
+    empty transcript, and sizes the GPU workspace as the reference does."""
+    k = load("refcpu_random_B4_T13_U6_V9.npz")
+    lp = k["log_probs"]
+    B, T, U, V = lp.shape
+    c, g = oracle.rnnt_cost_and_grad(lp, k["labels"], k["input_lengths"], k["label_lengths"], int(k["blank"]))
+    assert np.allclose(c, k["costs"], rtol=1e-6) and np.allclose(g, k["grads"], rtol=1e-5, atol=1e-7)
+    assert oracle.get_workspace_size(T, U, B, True) == (0, int(k["gpu_workspace_bytes"]))
 
 
 def test_invalid_arguments(oracle):
@@ -135,50 +132,27 @@ def test_invalid_arguments(oracle):
 
 
 def test_against_live_reference_property(oracle):
-    """Property-based pin (hypothesis, fixed seed database off): on random shapes, ragged lengths, blank positions and
-    logit scales the restatement and the unmodified reference library agree on costs and log-prob gradients."""
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref/libwarprnnt.so not available")
-    from hypothesis import given, settings, strategies as st, HealthCheck
-
-    @settings(max_examples=40, deadline=None, derandomize=True, database=None,
-              suppress_health_check=[HealthCheck.too_slow, HealthCheck.data_too_large])
-    @given(st.integers(1, 4), st.integers(1, 12), st.integers(1, 7), st.integers(2, 11), st.integers(0, 2 ** 31 - 1),
-           st.sampled_from([0.3, 1.0, 6.0]))
-    def run(B, T, U, V, seed, scale):
-        rng = np.random.default_rng(seed)
-        acts = (scale * rng.standard_normal((B, T, U, V))).astype(np.float32)
-        blank = int(rng.integers(0, V))
-        cand = np.array([v for v in range(V) if v != blank])
-        labels = (rng.choice(cand, size=(B, U - 1)).astype(np.int32) if U > 1 else np.zeros((B, 0), np.int32))
-        il = rng.integers(1, T + 1, B).astype(np.int32)
-        ll = rng.integers(0, U, B).astype(np.int32)
-        il[0], ll[0] = T, U - 1                       # the reference sizes its slabs by maxT / maxU
-        lp = oracle.log_softmax(acts)
-        c, g = oracle.rnnt_cost_and_grad(lp, labels, il, ll, blank=blank)
-        cr, gr = oracle.ref_cpu_cost_and_grad(lp, labels, il, ll, blank=blank, num_threads=1)
-        assert np.allclose(c, cr, rtol=1e-5, atol=1e-6), (B, T, U, V, seed)
-        assert np.allclose(g, gr, rtol=1e-4, atol=1e-6), (B, T, U, V, seed)
-
-    run()
+    """Property-based pin: on the 40 random shapes, ragged lengths, blank positions and logit scales that hypothesis drew
+    (tests/golden/make_golden.py: PROPERTY_CASES) the restatement and the unmodified reference library agree on costs
+    and log-prob gradients."""
+    cases = load_cases("refcpu_property_cases.npz")
+    assert len(cases) == 40
+    for k in cases:
+        lp, blank = k["log_probs"], int(k["blank"])
+        c, g = oracle.rnnt_cost_and_grad(lp, k["labels"], k["input_lengths"], k["label_lengths"], blank=blank)
+        assert np.allclose(c, k["costs"], rtol=1e-5, atol=1e-6), (lp.shape, blank)
+        assert np.allclose(g, k["grads"], rtol=1e-4, atol=1e-6), (lp.shape, blank)
 
 
 def test_joint_oracle_against_torch_fp64_chain_property(oracle):
     """The joint is parity-unpinned by the reference (TensorFlow arithmetic): its anchor is model.py:158-166 restated in
     torch fp64 and chained by autograd through log_softmax into the reference library's fp64 entry point
-    (tests/golden/make_golden.py: joint_case).  Fresh random shapes here, beyond the committed fixtures."""
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref/libwarprnnt.so not available")
-    import importlib.util
-    import os
-    spec = importlib.util.spec_from_file_location("make_golden", os.path.join(os.path.dirname(__file__), "golden", "make_golden.py"))
-    mg = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mg)
-    rng = np.random.default_rng(20260924)
-    for _ in range(10):
-        B, T, U = int(rng.integers(1, 4)), int(rng.integers(1, 9)), int(rng.integers(1, 6))
-        V, H = int(rng.integers(2, 9)), int(rng.integers(1, 7))
-        k = mg.joint_case(rng, B, T, U, V, H, blank=int(rng.integers(0, V)), ragged=bool(rng.integers(0, 2)))
+    (tests/golden/make_golden.py: joint_case).  Ten random shapes here, beyond the named joint fixtures."""
+    cases = load_cases("jointchain_property_cases.npz")
+    assert len(cases) == 10
+    for k in cases:
+        B, T, H = k["enc"].shape
+        U, V = k["pred"].shape[1], k["W"].shape[1]
         o64 = oracle.joint_loss_grad(*(k[n].astype(np.float64) for n in ("enc", "pred", "W", "b")), k["labels"],
                                      k["input_lengths"], k["label_lengths"], int(k["blank"]), grad_scale=np.full(B, 1.0 / B))
         assert np.allclose(o64["costs"], k["costs"], rtol=1e-10), (B, T, U, V, H)
