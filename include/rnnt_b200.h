@@ -133,14 +133,19 @@ rnntStatus_t rnntb200_loss_device(const float* activations, float* gradients, co
 typedef enum {
     RNNTB200_FP32_EXACT = 0, /**< fp32 CUDA-core arithmetic; parity gate rtol 1e-4 (BASELINE C1/C2) */
     RNNTB200_BF16_TC = 1     /**< 16-bit operands on tcgen05 tensor cores, fp32 accumulate (BASELINE C3-C5): the forward
-                                  projection runs on fp16 z / W (11-bit significands), the two gradient GEMMs on bf16 */
+                                  projection runs on fp16 z / W (11-bit significands), the two gradient GEMMs on bf16.
+                                  Any V >= 1 and 1 <= H <= 768: the kernels run the problem padded to Hp = ceil64(H),
+                                  Vp = ceil64(V), padding that contributes exactly zero (zero W / enc / pred columns, bias
+                                  -inf for v >= V); inputs and outputs keep their unpadded shapes */
 } rnntb200Precision;
 
 /** Problem descriptor of the fused joint + loss path (model.py:158-166 hoisted form, SURVEY 8a2):
  *    z[b,t,u,:]  = tanh(enc[b,t,:] + pred[b,u,:])            model.py:158-163
  *    logits      = z . W + bias,  W is (H,V) row-major        model.py:165-166
  *    costs[b]    = RNN-T NLL of logits[b] (softmax inside)    utils/loss.py:24-36
- *  RNNTB200_BF16_TC requires H % 64 == 0, 64 <= H <= 768 and V % 64 == 0. */
+ *  RNNTB200_BF16_TC takes any V >= 1 and 1 <= H <= 768 (H > 768: RNNT_STATUS_INVALID_VALUE, use RNNTB200_FP32_EXACT).
+ *  Its workspace is that of the padded problem (ceil64(H), ceil64(V)); when H % 64 != 0 it also holds zero-padded copies
+ *  of enc and pred (written by the forward, read by the backward) and d_enc at the padded width. */
 typedef struct {
     int B, maxT, maxU, H, V;
     int blank_label;

@@ -45,7 +45,7 @@ constexpr int DW_NRS = 8;            // depth of the row-scale ring (K steps): t
 struct BwdParams {
     const float* enc; const float* pred;
     const int* xlen; const int* ylen;
-    int maxT, maxU, H, V;
+    int maxT, maxU, H, V;       // H, V: the padded Hp, Vp (enc / pred / d_enc rows are Hp wide, the kept rows Vp)
     int nTb, nUb, b0, nb;
     const int* slot;            // tile -> row block of the kept arrays (-1: tile outside the valid lattice)
     const int* tile_of_slot;    // inverse map (valid tiles only)
@@ -442,13 +442,16 @@ __global__ void __launch_bounds__(DZ_THREADS, 1) bwd_dz_kernel(const __grid_cons
     }
 }
 
-// d_pred[b,u,:] = sum over the t-blocks that intersect the utterance of its partial planes (0 for u >= U_b)
+// d_pred[b,u,:] = sum over the t-blocks that intersect the utterance of its partial planes (0 for u >= U_b).  The planes
+// are Hp = 4 * H4 wide; d_pred (B, maxU, H) receives the first H columns of each row.
 __global__ void __launch_bounds__(256) sum_pred_planes_kernel(const float4* __restrict__ ppred, const int* __restrict__ xlen,
                                                               const int* __restrict__ ylen, int b0, int nb, int maxU, int H4,
-                                                              float4* __restrict__ d_pred) {
+                                                              int H, float* __restrict__ d_pred) {
     const size_t n4 = (size_t)nb * maxU * H4;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
         const int bl = (int)(i / ((size_t)maxU * H4)), u = (int)((i / H4) % maxU), b = b0 + bl;
+        const int h = (int)(i % H4) * 4;
+        if (h >= H) continue;                   // padding columns of the planes
         float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
         if (u < ylen[b] + 1) {
             const int ntb = (xlen[b] + BW_TT - 1) / BW_TT;
@@ -458,7 +461,15 @@ __global__ void __launch_bounds__(256) sum_pred_planes_kernel(const float4* __re
                 acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
             }
         }
-        d_pred[(size_t)b0 * maxU * H4 + i] = acc;
+        if (H == 4 * H4) {
+            reinterpret_cast<float4*>(d_pred)[(size_t)b0 * maxU * H4 + i] = acc;
+        } else {
+            float* o = d_pred + ((size_t)b0 * maxU + i / H4) * H + h;
+            o[0] = acc.x;
+            if (h + 1 < H) o[1] = acc.y;
+            if (h + 2 < H) o[2] = acc.z;
+            if (h + 3 < H) o[3] = acc.w;
+        }
     }
 }
 

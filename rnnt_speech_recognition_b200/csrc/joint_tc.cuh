@@ -4,6 +4,11 @@
 // contractions).  One persistent CTA per SM, each looping over 128-cell lattice tiles (16 time steps x 8 label positions
 // of one utterance); the (B,T,U,H) activation tensor of model.py:158-163 and the (B,T,U,V) logits of model.py:165-166
 // never exist in HBM.
+//
+// Any 1 <= H <= 768 and any V >= 1: the kernels always work on the PADDED problem Hp = ceil64(H), Vp = ceil64(V), whose
+// padding contributes exactly zero -- W^T / W are converted into zero-padded (Vp, Hp) / (Hp, Vp) operands, a column v >= V
+// gets the bias -inf (numerator 0), and when H % 64 != 0 enc / pred are staged into zero-padded (rows, Hp) arrays and d_enc
+// is accumulated at width Hp and narrowed once.  Aligned shapes run exactly the launches they always did.
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -24,6 +29,15 @@ namespace rb {
 
 constexpr int TC_MAX_KB = 16;        // H <= 1024
 constexpr int TC_TMEM_COLS = 512;
+
+// the tensor-core kernels' granularity along H and V: every problem is run at (ceil64(H), ceil64(V))
+inline int tc_pad64(int x) { return (x + 63) / 64 * 64; }
+inline rnntb200JointDesc tc_padded(const rnntb200JointDesc& d) {
+    rnntb200JointDesc p = d;
+    p.H = tc_pad64(d.H);
+    p.V = tc_pad64(d.V);
+    return p;
+}
 
 struct TcGeom {
     int TT, UU, nTb, nUb;  // tile = TT x UU cells (TT*UU == 128); tiles per utterance
@@ -119,7 +133,8 @@ inline BwdGeom bwd_geometry(int H, int V, int sms = 148, bool dz_pair = true, bo
 struct JointTcParams {
     const float* enc; const float* pred; const float* bias;
     const int* labels; const int* xlen; const int* ylen;
-    int B, maxT, maxU, H, V, blank;
+    int B, maxT, maxU, H, V, blank;   // H: the padded width Hp (enc / pred rows as the kernel reads them); V: the REAL vocabulary
+    int Vp;                           // ceil64(V): columns of W^T, of the kept rows and of the bias table; v >= V is masked (bias -inf)
     int TT, UU, nTb, nUb, NC, NCH, KB, stages;
     long long SK;
     int b0, nb;                 // utterance range of this launch
@@ -145,9 +160,10 @@ __device__ __forceinline__ TileInfo decode_tile(const JointTcParams& p, int tile
     return ti;
 }
 
-// W (H,V) fp32 -> Wt (V,H) fp16 [B operand of the logits GEMM, K=h] and Wb (H,V) bf16 [B operand of dZ, K=v]
+// W (H,V) fp32 -> Wt (Vp,Hp) fp16 [B operand of the logits GEMM, K=h] and Wb (Hp,Vp) bf16 [B operand of dZ, K=v], zero
+// outside (H, V); grid (Vp / 32, Hp / 32)
 __global__ void __launch_bounds__(256) convert_w_kernel(const float* __restrict__ W, __nv_bfloat16* __restrict__ Wt,
-                                                        __nv_bfloat16* __restrict__ Wb, int H, int V) {
+                                                        __nv_bfloat16* __restrict__ Wb, int H, int V, int Hp, int Vp) {
     __shared__ float tile[32][33];
     const int v0 = blockIdx.x * 32, h0 = blockIdx.y * 32;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
@@ -155,12 +171,37 @@ __global__ void __launch_bounds__(256) convert_w_kernel(const float* __restrict_
         const int h = h0 + i, v = v0 + tx;
         const float w = (h < H && v < V) ? W[(size_t)h * V + v] : 0.f;
         tile[i][tx] = w;
-        if (h < H && v < V) Wb[(size_t)h * V + v] = __float2bfloat16(w);
+        if (h < Hp && v < Vp) Wb[(size_t)h * Vp + v] = __float2bfloat16(w);
     }
     __syncthreads();
     for (int i = ty; i < 32; i += 8) {
         const int v = v0 + i, h = h0 + tx;
-        if (h < H && v < V) reinterpret_cast<__half*>(Wt)[(size_t)v * H + h] = __float2half_rn(tile[tx][i]);
+        if (h < Hp && v < Vp) reinterpret_cast<__half*>(Wt)[(size_t)v * Hp + h] = __float2half_rn(tile[tx][i]);
+    }
+}
+
+// H % 64 != 0: enc (rows_e, H) and pred (rows_p, H) -> zero-padded (rows, Hp) copies in the workspace, one launch.  The
+// caller's rows cannot be read in place: TMA needs 16-byte row strides and the dZ epilogue adds d_enc as float4.
+__global__ void __launch_bounds__(256) stage_rows_kernel(const float* __restrict__ enc, const float* __restrict__ pred,
+                                                         float* __restrict__ enc_s, float* __restrict__ pred_s,
+                                                         long long rows_e, long long rows_p, int H, int Hp) {
+    const long long ne = rows_e * Hp, n = (rows_e + rows_p) * Hp;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const bool is_e = i < ne;
+        const long long j = is_e ? i : i - ne, r = j / Hp;
+        const int h = (int)(j - r * Hp);
+        const float x = h < H ? (is_e ? enc : pred)[r * H + h] : 0.f;
+        (is_e ? enc_s : pred_s)[j] = x;
+    }
+}
+
+// out (rows, H) = the first H columns of src (rows, Hp): d_enc accumulated at the padded width
+__global__ void __launch_bounds__(256) narrow_rows_kernel(const float* __restrict__ src, long long rows, int Hp, int H,
+                                                          float* __restrict__ out) {
+    const long long n = rows * H;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const long long r = i / H;
+        out[i] = src[r * Hp + (i - r * H)];
     }
 }
 
@@ -222,17 +263,34 @@ __global__ void __launch_bounds__(1024) tile_compact_kernel(const int* __restric
                    base, max_slots);
     }
 }
-// out[i] = sum_k part[k][i] over `nplanes` planes of `n4` float4 each
+// out = sum_k part[k] over `nplanes` planes of `n4` float4 each; a plane is (rows, 4 * cols4) and out receives its
+// window (rows_out, cols_out) -- the real (H, V) of a padded (Hp, Vp) plane -- as a dense row-major array
 __global__ void __launch_bounds__(256) sum_planes_kernel(const float4* __restrict__ part, int nplanes, size_t n4,
-                                                         float4* __restrict__ out) {
+                                                         float* __restrict__ out, int rows_out, int cols4, int cols_out) {
+    const bool whole = cols_out == 4 * cols4 && (size_t)rows_out * cols4 == n4;      // aligned: the window is the whole plane
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
+        size_t r = 0;
+        int c = 0;
+        if (!whole) {
+            r = i / cols4;
+            c = (int)(i - r * cols4) * 4;
+            if (r >= (size_t)rows_out || c >= cols_out) continue;
+        }
         float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll 4
         for (int k = 0; k < nplanes; ++k) {
             const float4 v = part[(size_t)k * n4 + i];
             acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
         }
-        out[i] = acc;
+        if (whole) {
+            reinterpret_cast<float4*>(out)[i] = acc;
+        } else {
+            float* o = out + r * cols_out + c;
+            o[0] = acc.x;
+            if (c + 1 < cols_out) o[1] = acc.y;
+            if (c + 2 < cols_out) o[2] = acc.z;
+            if (c + 3 < cols_out) o[3] = acc.w;
+        }
     }
 }
 // ------------------------------------------------------------------------------------------
@@ -296,10 +354,12 @@ inline bool make_tmap_f32(CUtensorMap* tm, const void* base, uint64_t rows, uint
 }
 
 // Workspace of the tensor-core path (a pure function of the descriptor).  The kept arrays (numerators + maxima) are
-// laid out per 128-row tile; the batch is processed in utterance chunks that keep them under ~16 GiB.
+// laid out per 128-row tile; the batch is processed in utterance chunks that keep them under ~16 GiB.  Every size below is
+// that of the padded problem (Hp, Vp) = (ceil64(H), ceil64(V)); the three staged arrays at the end exist only when H != Hp,
+// so an aligned descriptor has exactly the layout it always had.
 struct TcScratch {
-    __nv_bfloat16 *Wt, *Wb;                 // W^T (V,H) fp16 [forward B operand, 16-bit storage] and W (H,V) bf16 [dZ B operand]
-    __nv_bfloat16* dl;                      // (rows_chunk, V) bf16 softmax numerators E = 2^(y - ref_row)
+    __nv_bfloat16 *Wt, *Wb;                 // W^T (Vp,Hp) fp16 [forward B operand, 16-bit storage] and W (Hp,Vp) bf16 [dZ B operand]
+    __nv_bfloat16* dl;                      // (rows_chunk, Vp) bf16 softmax numerators E = 2^(y - ref_row)
     float* gm;                              // (rows_chunk) fp32 reference of each row's numerators (log2 domain)
     int* slot;                              // tile -> compact row block (-1: outside the valid lattice), per chunk
     int* tile_of_slot;                      // compact row block -> tile
@@ -309,6 +369,8 @@ struct TcScratch {
     float* dWp;                             // (S_max, H, V) fp32 split-K planes of dW (bwd_dw_kernel)
     float* dbp;                             // (S_max, V) planes of db
     float* rowscale;                        // (rows_chunk) per-row scale of the logit gradients (row_scale_kernel)
+    float *enc_s, *pred_s;                  // H != Hp only: (B*maxT, Hp) / (B*maxU, Hp) zero-padded copies of enc / pred
+    float* denc_s;                          // H != Hp only: (B*maxT, Hp) d_enc at the padded width, narrowed at the end
     int bchunk;                             // utterances per chunk
     size_t rows_chunk;                      // bchunk * tiles_per_utt * 128
     size_t bytes;
@@ -320,8 +382,9 @@ inline size_t tc_chunk_budget() {
     if (!v) { const char* e = getenv("RNNTB200_CHUNK_MB"); v = e && atoll(e) > 0 ? (size_t)atoll(e) << 20 : (size_t)16 << 30; }
     return v;
 }
-inline TcScratch tc_scratch_layout(const rnntb200JointDesc& d, void* base) {
+inline TcScratch tc_scratch_layout(const rnntb200JointDesc& desc, void* base) {
     TcScratch s{};
+    const rnntb200JointDesc d = tc_padded(desc);
     const TcGeom g = tc_geometry(d.maxT, d.maxU, d.H, d.V);
     const BwdGeom bg = bwd_geometry(d.H, d.V, 148, tc_dz_variant() == 2, tc_dw_variant() == 2);
     const size_t rows_utt = (size_t)g.nTb * g.nUb * 128;
@@ -353,14 +416,18 @@ inline TcScratch tc_scratch_layout(const rnntb200JointDesc& d, void* base) {
     s.dWp = reinterpret_cast<float*>(take((size_t)bg.S_max * d.H * d.V * 4));
     s.dbp = reinterpret_cast<float*>(take((size_t)bg.S_max * d.V * 4));
     s.rowscale = reinterpret_cast<float*>(take(s.rows_chunk * 4));
+    if (desc.H != d.H) {
+        s.enc_s = reinterpret_cast<float*>(take((size_t)d.B * d.maxT * d.H * 4));
+        s.pred_s = reinterpret_cast<float*>(take((size_t)d.B * d.maxU * d.H * 4));
+        s.denc_s = reinterpret_cast<float*>(take((size_t)d.B * d.maxT * d.H * 4));
+    }
     s.bytes = (size_t)(p - static_cast<char*>(base));
     return s;
 }
 
 inline rnntStatus_t tc_unsupported(const rnntb200JointDesc& d) {
     fprintf(stderr,
-            "rnnt_b200: RNNTB200_BF16_TC needs H %% 64 == 0, V %% 64 == 0 and 64 <= H <= 768 (got H=%d V=%d); "
-            "use RNNTB200_FP32_EXACT\n", d.H, d.V);
+            "rnnt_b200: RNNTB200_BF16_TC supports joint widths H <= 768 (got H=%d); use RNNTB200_FP32_EXACT\n", d.H);
     return RNNT_STATUS_INVALID_VALUE;
 }
 
@@ -369,7 +436,7 @@ inline bool tc_fill_params(const rnntb200JointDesc& d, const TcGeom& g, JointTcP
                            const int* xlen) {
     p = JointTcParams{};
     p.enc = enc; p.pred = pred; p.bias = bias; p.labels = labels; p.xlen = xlen; p.ylen = ylen;
-    p.B = d.B; p.maxT = d.maxT; p.maxU = d.maxU; p.H = d.H; p.V = d.V; p.blank = d.blank_label;
+    p.B = d.B; p.maxT = d.maxT; p.maxU = d.maxU; p.H = tc_pad64(d.H); p.V = d.V; p.Vp = tc_pad64(d.V); p.blank = d.blank_label;
     p.TT = g.TT; p.UU = g.UU; p.nTb = g.nTb; p.nUb = g.nUb; p.KB = g.KB;
     p.SK = (long long)(d.maxT + d.maxU - 1) * d.maxU;
     return true;
@@ -420,7 +487,10 @@ inline long long* tc_prof_buffer(int which) {
     return buf[which];
 }
 
-inline bool tc_supported(const rnntb200JointDesc& d) {
+// 1 <= H <= 768 and V >= 1: the geometries are those of the padded problem
+inline bool tc_supported(const rnntb200JointDesc& desc) {
+    if (desc.H < 1 || desc.H > 768 || desc.V < 1) return false;
+    const rnntb200JointDesc d = tc_padded(desc);
     return tc_geometry(d.maxT, d.maxU, d.H, d.V).ok && tc3_geometry(d.H, d.V).ok && bwd_geometry(d.H, d.V, 148, tc_dz_variant() == 2, tc_dw_variant() == 2).ok;
 }
 inline size_t tc_scratch_bytes(const rnntb200JointDesc& d) {
@@ -451,12 +521,13 @@ inline rnntStatus_t tc_run_forward(const rnntb200JointDesc& d, const TcGeom& g, 
                                    const int* xlen, float* lse, float* lpb, float* lpl, int b0, int nb, cudaStream_t s,
                                    unsigned* launches) {
     const bool pair = tc_fwd_variant() == 4;             // CTA-pair kernel (joint_tc4.cuh) or one CTA per tile (joint_tc3.cuh)
-    const Tc2Geom g3 = pair ? tc4_geometry(d.H, d.V) : tc3_geometry(d.H, d.V);
+    const int Hp = tc_pad64(d.H), Vp = tc_pad64(d.V);    // enc / pred are (rows, Hp) here: the caller's or the staged copies
+    const Tc2Geom g3 = pair ? tc4_geometry(Hp, Vp) : tc3_geometry(Hp, Vp);
     JointTcParams p;
     tc_fill_params(d, g, p, enc, pred, bias, labels, ylen, xlen);
     p.b0 = b0; p.nb = nb;
     p.lse = lse; p.lpb = lpb; p.lpl = lpl;
-    p.NC = TC2_NC; p.NCH = d.V / TC2_NC; p.stages = g3.stages; p.nbuf = g3.nbuf; p.ks = g3.ks;
+    p.NC = TC2_NC; p.NCH = Vp / TC2_NC; p.stages = g3.stages; p.nbuf = g3.nbuf; p.ks = g3.ks;
     p.dbg = tc_dbg();
     if (KEEP) {
         const int ntiles = nb * g.nTb * g.nUb;
@@ -466,9 +537,9 @@ inline rnntStatus_t tc_run_forward(const rnntb200JointDesc& d, const TcGeom& g, 
         p.slot = sc.slot; p.dl = sc.dl; p.gm = sc.gm;
     }
     CUtensorMap tm, tmp, tme;
-    if (!make_tmap_bf16_kblocks(&tm, sc.Wt, d.V, d.H, pair ? TC2_NC / 2 : TC2_NC, g3.ks) ||
-        !make_tmap_f32(&tmp, pred, (uint64_t)d.B * d.maxU, d.H, g.UU, 32, true) ||
-        !make_tmap_f32(&tme, enc, (uint64_t)d.B * d.maxT, d.H, g.TT, 64, false)) {
+    if (!make_tmap_bf16_kblocks(&tm, sc.Wt, Vp, Hp, pair ? TC2_NC / 2 : TC2_NC, g3.ks) ||
+        !make_tmap_f32(&tmp, pred, (uint64_t)d.B * d.maxU, Hp, g.UU, 32, true) ||
+        !make_tmap_f32(&tme, enc, (uint64_t)d.B * d.maxT, Hp, g.TT, 64, false)) {
         fprintf(stderr, "rnnt_b200: cuTensorMapEncodeTiled failed\n");
         return RNNT_STATUS_EXECUTION_FAILED;
     }
@@ -482,10 +553,19 @@ inline rnntStatus_t tc_forward(const rnntb200JointDesc& d, void* scratch, const 
                                const int* xlen, float* lse, float* lpb, float* lpl, cudaStream_t s,
                                unsigned* launches) {
     if (!tc_supported(d)) return tc_unsupported(d);
-    const TcGeom g = tc_geometry(d.maxT, d.maxU, d.H, d.V);
+    const rnntb200JointDesc dp = tc_padded(d);
+    const TcGeom g = tc_geometry(dp.maxT, dp.maxU, dp.H, dp.V);
     TcScratch sc = tc_scratch_layout(d, scratch);
-    convert_w_kernel<<<dim3((d.V + 31) / 32, (d.H + 31) / 32), 256, 0, s>>>(W, sc.Wt, sc.Wb, d.H, d.V);
+    convert_w_kernel<<<dim3(dp.V / 32, dp.H / 32), 256, 0, s>>>(W, sc.Wt, sc.Wb, d.H, d.V, dp.H, dp.V);
     *launches += 1;
+    if (dp.H != d.H) {      // the backward reads these copies too (it follows the forward with the same workspace)
+        const long long re = (long long)d.B * d.maxT, rp = (long long)d.B * d.maxU, n = (re + rp) * dp.H;
+        stage_rows_kernel<<<(unsigned)((n + 255) / 256 < 4096 ? (n + 255) / 256 : 4096), 256, 0, s>>>(enc, pred, sc.enc_s, sc.pred_s,
+                                                                                                   re, rp, d.H, dp.H);
+        *launches += 1;
+        enc = sc.enc_s;
+        pred = sc.pred_s;
+    }
     if (tc_keep(d, sc))
         return tc_run_forward<true>(d, g, sc, enc, pred, bias, labels, ylen, xlen, lse, lpb, lpl, 0, d.B, s, launches);
     return tc_run_forward<false>(d, g, sc, enc, pred, bias, labels, ylen, xlen, lse, lpb, lpl, 0, d.B, s, launches);
@@ -502,25 +582,29 @@ inline rnntStatus_t tc_backward(const rnntb200JointDesc& d, void* scratch, const
                                 const LossPlanes& lp, const float* grad_costs, float* d_enc, float* d_pred, float* dW,
                                 float* db, cudaStream_t s, unsigned* launches) {
     if (!tc_supported(d)) return tc_unsupported(d);
-    const TcGeom g = tc_geometry(d.maxT, d.maxU, d.H, d.V);
+    const rnntb200JointDesc dp = tc_padded(d);
+    const int Hp = dp.H, Vp = dp.V;
+    const TcGeom g = tc_geometry(dp.maxT, dp.maxU, Hp, Vp);
     const bool dz_pair = tc_dz_variant() == 2, dw_pair = tc_dw_variant() == 2;
-    const BwdGeom bg = bwd_geometry(d.H, d.V, 148, dz_pair, dw_pair);
-    TcScratch sc = tc_scratch_layout(d, scratch);   // Wt / Wb were produced by the forward call
+    const BwdGeom bg = bwd_geometry(Hp, Vp, 148, dz_pair, dw_pair);
+    TcScratch sc = tc_scratch_layout(d, scratch);   // Wt / Wb (and for H != Hp the staged enc / pred) were produced by the forward call
     const bool kept = tc_keep(d, sc);
+    float* d_enc_out = d_enc;
+    if (Hp != d.H) { enc = sc.enc_s; pred = sc.pred_s; d_enc = sc.denc_s; }
     if (!tc_smem_optin(reinterpret_cast<const void*>(bwd_dz_kernel<false, false>)) || !tc_smem_optin(reinterpret_cast<const void*>(bwd_dz_kernel<true, false>)) ||
         !tc_smem_optin(reinterpret_cast<const void*>(bwd_dz_kernel<false, true>)) || !tc_smem_optin(reinterpret_cast<const void*>(bwd_dz_kernel<true, true>)) ||
         !tc_smem_optin(reinterpret_cast<const void*>(bwd_dw_kernel<false>)) || !tc_smem_optin(reinterpret_cast<const void*>(bwd_dw_kernel<true>)) ||
         !tc_smem_optin(reinterpret_cast<const void*>(bwd_dw2_kernel<false>)) || !tc_smem_optin(reinterpret_cast<const void*>(bwd_dw2_kernel<true>)))
         return RNNT_STATUS_EXECUTION_FAILED;
-    if (cudaMemsetAsync(sc.dWp, 0, sizeof(float) * (size_t)bg.S_max * d.H * d.V, s) != cudaSuccess ||
-        cudaMemsetAsync(sc.dbp, 0, sizeof(float) * (size_t)bg.S_max * d.V, s) != cudaSuccess)
+    if (cudaMemsetAsync(sc.dWp, 0, sizeof(float) * (size_t)bg.S_max * Hp * Vp, s) != cudaSuccess ||
+        cudaMemsetAsync(sc.dbp, 0, sizeof(float) * (size_t)bg.S_max * Vp, s) != cudaSuccess)
         return RNNT_STATUS_MEMOPS_FAILED;
     CUtensorMap tm_e128, tm_e64, tm_wp, tm_ws, tm_p32, tm_e32;
-    if (!make_tmap_f32(&tm_p32, pred, (uint64_t)d.B * d.maxU, d.H, BW_UU, 32, true) ||
-        !make_tmap_f32(&tm_e32, enc, (uint64_t)d.B * d.maxT, d.H, BW_TT, 32, false) ||
-        !make_tmap_bf16(&tm_e128, sc.dl, sc.rows_chunk, d.V, 128) || !make_tmap_bf16(&tm_e64, sc.dl, sc.rows_chunk, d.V, 64) ||
-        !make_tmap_bf16(&tm_wp, sc.Wb, d.H, d.V, dz_pair ? bg.priv / 2 : bg.priv) ||
-        !make_tmap_bf16(&tm_ws, sc.Wb, d.H, d.V, bg.sh ? (dz_pair ? bg.sh / 2 : bg.sh) : 8)) {
+    if (!make_tmap_f32(&tm_p32, pred, (uint64_t)d.B * d.maxU, Hp, BW_UU, 32, true) ||
+        !make_tmap_f32(&tm_e32, enc, (uint64_t)d.B * d.maxT, Hp, BW_TT, 32, false) ||
+        !make_tmap_bf16(&tm_e128, sc.dl, sc.rows_chunk, Vp, 128) || !make_tmap_bf16(&tm_e64, sc.dl, sc.rows_chunk, Vp, 64) ||
+        !make_tmap_bf16(&tm_wp, sc.Wb, Hp, Vp, dz_pair ? bg.priv / 2 : bg.priv) ||
+        !make_tmap_bf16(&tm_ws, sc.Wb, Hp, Vp, bg.sh ? (dz_pair ? bg.sh / 2 : bg.sh) : 8)) {
         fprintf(stderr, "rnnt_b200: cuTensorMapEncodeTiled failed\n");
         return RNNT_STATUS_EXECUTION_FAILED;
     }
@@ -533,24 +617,24 @@ inline rnntStatus_t tc_backward(const rnntb200JointDesc& d, void* scratch, const
         }
         BwdParams p{};
         p.enc = enc; p.pred = pred; p.xlen = xlen; p.ylen = ylen;
-        p.maxT = d.maxT; p.maxU = d.maxU; p.H = d.H; p.V = d.V;
+        p.maxT = d.maxT; p.maxU = d.maxU; p.H = Hp; p.V = Vp;
         p.nTb = g.nTb; p.nUb = g.nUb; p.b0 = b0; p.nb = nb;
         {   // per-row scales of this chunk (row order of the kept arrays) + the two special columns of every row
             ScopedTimer tmr("row_scale_kernel", s);
             row_scale_kernel<<<(unsigned)(((size_t)nb * g.nTb * g.nUb * 128 + 255) / 256), 256, 0, s>>>(
                 sc.tile_of_slot, sc.count, b0, g.nTb, g.nUb, xlen, ylen, labels, d.blank_label, d.maxT, d.maxU,
                 (long long)(d.maxT + d.maxU - 1) * d.maxU, lp.lse, lp.lpb, lp.lpl, lp.alphas, lp.betas, lp.llf, grad_costs, sc.gm,
-                d.V, reinterpret_cast<unsigned short*>(sc.dl), sc.rowscale);
+                Vp, reinterpret_cast<unsigned short*>(sc.dl), sc.rowscale);
             *launches += 1;
         }
         p.slot = sc.slot; p.tile_of_slot = sc.tile_of_slot; p.slot_meta = sc.slot_meta; p.count = sc.count; p.rowscale = sc.rowscale;
         p.NP = bg.NP; p.NCZ = bg.NCZ; p.priv = bg.priv; p.sh = bg.sh; p.odd_base = bg.odd_base; p.dz_stages = bg.dz_stages;
         p.d_enc = d_enc; p.ppred = sc.ppl;
-        p.nVT = bg.nVT; p.nItems = bg.nItems; p.nHB = bg.nHB; p.S = bg.S_max; p.Hrows = d.H;
+        p.nVT = bg.nVT; p.nItems = bg.nItems; p.nHB = bg.nHB; p.S = bg.S_max; p.Hrows = Hp;
         p.dWp = sc.dWp; p.dbp = sc.dbp;
         long long* prof_dz = tc_prof_buffer(0), *prof_dw = tc_prof_buffer(1);
         // rows of d_enc whose t-block lies outside the utterance are never visited by the dZ kernel
-        if (cudaMemsetAsync(d_enc + (size_t)b0 * d.maxT * d.H, 0, sizeof(float) * (size_t)nb * d.maxT * d.H, s) != cudaSuccess)
+        if (cudaMemsetAsync(d_enc + (size_t)b0 * d.maxT * Hp, 0, sizeof(float) * (size_t)nb * d.maxT * Hp, s) != cudaSuccess)
             return RNNT_STATUS_MEMOPS_FAILED;
         {
             const int nruns = nb * g.nTb;
@@ -571,10 +655,10 @@ inline rnntStatus_t tc_backward(const rnntb200JointDesc& d, void* scratch, const
             else bwd_dz_kernel<false, false><<<nruns < sms ? nruns : sms, DZ_THREADS, bg.dz_smem, s>>>(tm_e128, tm_wp, tm_ws, tm_p32, tm_e32, p);
         }
         {
-            const size_t n4 = (size_t)nb * d.maxU * d.H / 4;
+            const size_t n4 = (size_t)nb * d.maxU * Hp / 4;
             ScopedTimer tmr("sum_pred_planes_kernel", s);
             sum_pred_planes_kernel<<<(unsigned)((n4 + 255) / 256 < 4096 ? (n4 + 255) / 256 : 4096), 256, 0, s>>>(
-                reinterpret_cast<const float4*>(sc.ppl), xlen, ylen, b0, nb, d.maxU, d.H / 4, reinterpret_cast<float4*>(d_pred));
+                reinterpret_cast<const float4*>(sc.ppl), xlen, ylen, b0, nb, d.maxU, Hp / 4, d.H, d_pred);
         }
         {
             ScopedTimer tmr(dw_pair ? "bwd_dw2_kernel" : "bwd_dw_kernel", s);
@@ -590,13 +674,19 @@ inline rnntStatus_t tc_backward(const rnntb200JointDesc& d, void* scratch, const
     }
     {
         ScopedTimer tmr("sum_planes_kernel", s);
-        const size_t nw4 = (size_t)d.H * d.V / 4, nb4 = (size_t)d.V / 4;
+        const size_t nw4 = (size_t)Hp * Vp / 4, nb4 = (size_t)Vp / 4;
         sum_planes_kernel<<<(unsigned)((nw4 + 255) / 256 < 4096 ? (nw4 + 255) / 256 : 4096), 256, 0, s>>>(
-            reinterpret_cast<const float4*>(sc.dWp), bg.S_max, nw4, reinterpret_cast<float4*>(dW));
+            reinterpret_cast<const float4*>(sc.dWp), bg.S_max, nw4, dW, d.H, Vp / 4, d.V);
         sum_planes_kernel<<<(unsigned)((nb4 + 255) / 256), 256, 0, s>>>(reinterpret_cast<const float4*>(sc.dbp), bg.S_max, nb4,
-                                                                       reinterpret_cast<float4*>(db));
+                                                                       db, 1, Vp / 4, d.V);
     }
     *launches += 2;
+    if (Hp != d.H) {
+        const long long n = (long long)d.B * d.maxT * d.H;
+        narrow_rows_kernel<<<(unsigned)((n + 255) / 256 < 4096 ? (n + 255) / 256 : 4096), 256, 0, s>>>(sc.denc_s, (long long)d.B * d.maxT,
+                                                                                                    Hp, d.H, d_enc_out);
+        *launches += 1;
+    }
     return cudaGetLastError() == cudaSuccess ? RNNT_STATUS_SUCCESS : RNNT_STATUS_EXECUTION_FAILED;
 }
 

@@ -60,10 +60,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC3_THREADS, 1) join
     uint64_t* in_full = acc_empty + TC2_MAX_NBUF;         // [TC3_IN_STAGES]  input TMA -> producers
     uint64_t* in_empty = in_full + TC3_IN_STAGES;         // [TC3_IN_STAGES]  producers -> input TMA
     uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(in_empty + TC3_IN_STAGES);
-    float* bias2 = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(bars) + 1024);   // bias * log2(e) for V <= 4096 (else read from global)
-    const bool bias_in_smem = p.V <= 4096;
+    float* bias2 = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(bars) + 1024);   // bias * log2(e) for Vp <= 4096 (else read from global)
+    const bool bias_in_smem = p.Vp <= 4096;
+    // a padding column v >= V gets the bias -inf: its numerator 2^(y - ref) is exactly 0 (ref, the maximum of the first 32
+    // logits, always includes column 0 and stays finite)
     if (bias_in_smem)
-        for (int i = threadIdx.x; i < p.V; i += TC3_THREADS) bias2[i] = __ldg(p.bias + i) * 1.4426950408889634f;
+        for (int i = threadIdx.x; i < p.Vp; i += TC3_THREADS) bias2[i] = i < p.V ? __ldg(p.bias + i) * 1.4426950408889634f : -CUDART_INF_F;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (threadIdx.x == 0) {
@@ -350,7 +352,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC3_THREADS, 1) join
                             y[4 * i + 2] = fmaf(__uint_as_float(v[4 * i + 2]), LOG2E, b4.z); y[4 * i + 3] = fmaf(__uint_as_float(v[4 * i + 3]), LOG2E, b4.w);
                         }
                     } else {
-                        const float bv = __ldg(p.bias + col0 + lane) * LOG2E;
+                        const float bv = col0 + lane < p.V ? __ldg(p.bias + col0 + lane) * LOG2E : -CUDART_INF_F;
 #pragma unroll
                         for (int i = 0; i < 32; ++i)
                             y[i] = fmaf(__uint_as_float(v[i]), LOG2E, __shfl_sync(0xffffffffu, bv, i));
@@ -394,7 +396,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC3_THREADS, 1) join
                             m2 = mn;
                         }
                         if (MODE == 2 && has_slot) {
-                            __nv_bfloat16* dst = p.dl + (rowbase + r) * p.V + col0;
+                            __nv_bfloat16* dst = p.dl + (rowbase + r) * p.Vp + col0;
                             ptx::st_global_256(dst, o);
                             ptx::st_global_256(dst + 16, o + 8);
                         }

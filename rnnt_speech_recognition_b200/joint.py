@@ -115,6 +115,8 @@ def joint_rnnt_loss(enc_acts, pred_acts, W, b, labels, input_lengths, label_leng
     """Per-utterance RNN-T NLL (B,) of logits = tanh(enc_acts[:,:,None]+pred_acts[:,None]) @ W + b,
     differentiable w.r.t. enc_acts, pred_acts, W, b -- without ever materialising (B,T,U,V).
     precision: 'bf16' = the tensor-core path (tcgen05, 16-bit operands, fp32 accumulate) or 'fp32' (exact CUDA-core path).
+    'bf16' takes any vocabulary size V >= 1 and joint width 1 <= H <= 768 (the kernels pad to multiples of 64 internally;
+    the gradients come back in the shapes of the inputs); H > 768 raises -- use 'fp32'.
     compact: accepted for compatibility and ignored -- ragged batches are compacted on the device, the library never
     synchronises with the host.
     keep_activations: None = automatically when a gradient is required (the forward then leaves its softmax
