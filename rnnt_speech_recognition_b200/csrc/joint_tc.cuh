@@ -141,9 +141,9 @@ struct JointTcParams {
     const int* slot;            // tile -> compact row block of the kept arrays (valid tiles only); NULL = tile order
     int nbuf, ks, dbg;          // TMEM accumulator buffers; K-blocks per W stage; bring-up switches
     float* lse; float* lpb; float* lpl;              // outputs (NULL: a recompute that only wants the kept activations)
-    // MODE 2 (forward that KEEPS its activations): dl receives the softmax numerators 2^(y - gm) as fp16, one row of V
-    // per lattice cell, gm the running maximum each 32-column group was taken against.
-    __nv_bfloat16* dl;          // (16-bit storage; the numerators are fp16)
+    // MODE 2 (forward that KEEPS its activations): dl receives the softmax numerators 2^(y - gm) as bf16, one row of Vp
+    // per lattice cell, gm the row's final frame (log2 domain), against which every numerator of the row is below 2^64.
+    __nv_bfloat16* dl;
     float* gm;
 };
 struct TileInfo { int b, t0, u0, Tn, Un; bool valid; };

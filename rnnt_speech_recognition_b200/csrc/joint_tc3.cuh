@@ -17,10 +17,12 @@
 // MODE 0  forward: lse + (blank, label) log-probs per cell; nothing else leaves the SM
 // MODE 2  forward that KEEPS its activations (rnntb200JointDesc.keep_activations, and the backward's per-chunk
 //         recompute): MODE 0 + the softmax numerators E[row, v] = 2^(y_v - ref_row) as bf16, all columns of a row against
-//         ONE reference ref_row = the maximum of the row's first 32 logits (bf16 keeps its 8 significant bits over the whole
-//         exponent range, so any reference works; the exponent is clamped at +100), and ref_row itself.  The logit
-//         gradients are then row_scale * E: the two backward GEMMs take E straight from TMA and apply the row scale in an
-//         epilogue (dZ) or to the regenerated A operand (dW) -- no per-element prologue.
+//         ONE frame ref_row, and ref_row itself.  ref_row is the maximum of the row's first 32 logits unless a later
+//         group reaches 2^64 against it; the row then moves its frame up (here to its running maximum, in joint_tc4 to
+//         that group's maximum) and rescales what it has already stored (tc_rescale_kept).  So every kept numerator is below 2^64 (bf16 keeps its 8 significant bits over
+//         the whole exponent range), and a row scale flushed to 0 below 1e-30 drops at most 1e-30 * 2^64 ~ 2e-11 of
+//         gradient.  The logit gradients are then row_scale * E: the two backward GEMMs take E straight from TMA and apply
+//         the row scale in an epilogue (dZ) or to the regenerated A operand (dW) -- no per-element prologue.
 #pragma once
 #include <cuda_fp16.h>
 #include "joint_tc.cuh"
@@ -62,6 +64,20 @@ inline Tc2Geom tc3_geometry(int H, int V) {
     g.smem_bytes = 1024 + in_bytes + (size_t)g.stages * g.ks * 8192 + 1024 + bias_bytes;
     g.ok = g.stages >= 2;
     return g;
+}
+
+// The row's frame moved up: multiply the n numerators it has already kept (n a multiple of 32, the row 32-byte aligned)
+// by f = 2^(old frame - new frame) < 1.  The calling thread stored them itself, so plain loads see them.
+__device__ __forceinline__ void tc_rescale_kept(__nv_bfloat16* row, int n, float f) {
+    uint4* q = reinterpret_cast<uint4*>(row);
+    for (int i = 0; i < n / 8; ++i) {
+        uint4 w = q[i];
+        uint32_t* x = reinterpret_cast<uint32_t*>(&w);
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+            x[j] = ptx::pack_bf16x2(__uint_as_float(x[j] << 16) * f, __uint_as_float(x[j] & 0xffff0000u) * f);
+        q[i] = w;
+    }
 }
 
 template <int MODE>
@@ -307,12 +323,13 @@ __global__ void __launch_bounds__(TC3_THREADS, 1) joint_tc3_kernel(const __grid_
                         for (int i = 1; i < 32; ++i) gm = fmaxf(gm, y[i]);
                         const float mn = fmaxf(m2, gm);
                         float acc = 0.f;
-                        // Both modes form the group's sum from 2^(y - ref) against the row's FIXED reference (the maximum of its first 32
-                        // logits), rescaled once per group into the running-maximum frame: identical arithmetic, hence identical costs,
-                        // whether or not the numerators are kept.  MODE 2 stores those numerators (bf16).
+                        // Both modes form the group's sum from 2^(y - ref) against the row's frame ref (the maximum of its first 32
+                        // logits until a group reaches 2^64 against it), rescaled once per group into the running-maximum frame:
+                        // identical arithmetic, hence identical costs, whether or not the numerators are kept.  MODE 2 stores
+                        // those numerators (bf16).
                         if (col0 == 0) ref = gm;
                         uint32_t o[16];
-                        if (gm - ref <= 100.f) {
+                        if (gm - ref <= 64.f) {
                             float accr = 0.f;
 #pragma unroll
                             for (int i = 0; i < 32; i += 2) {
@@ -322,14 +339,17 @@ __global__ void __launch_bounds__(TC3_THREADS, 1) joint_tc3_kernel(const __grid_
                             }
                             acc = accr * ptx::ex2_approx(ref - mn);
                         } else {
-                            // a logit more than 2^100 above the reference (never seen outside adversarial inputs): the sum is taken
-                            // against the running maximum, the stored values are clamped at 2^100
+                            // a logit more than 64 bits above the frame (a confident row whose maximum lies beyond its first 32
+                            // columns): the row's frame moves up to the running maximum, which this group's numerators and the sum are
+                            // taken against; the numerators kept so far are brought into the new frame
 #pragma unroll
                             for (int i = 0; i < 32; i += 2) {
-                                acc += ptx::ex2_approx(y[i] - mn) + ptx::ex2_approx(y[i + 1] - mn);
-                                if (MODE == 2)
-                                    o[i >> 1] = ptx::pack_bf16x2(ptx::ex2_approx(fminf(y[i] - ref, 100.f)), ptx::ex2_approx(fminf(y[i + 1] - ref, 100.f)));
+                                const float e0 = ptx::ex2_approx(y[i] - mn), e1 = ptx::ex2_approx(y[i + 1] - mn);
+                                acc += e0 + e1;
+                                if (MODE == 2) o[i >> 1] = ptx::pack_bf16x2(e0, e1);
                             }
+                            if (MODE == 2 && has_slot) tc_rescale_kept(p.dl + (rowbase + r) * p.Vp, col0, ptx::ex2_approx(ref - mn));
+                            ref = mn;
                         }
                         if (MODE == 2 && has_slot) {
                             __nv_bfloat16* dst = p.dl + (rowbase + r) * p.Vp + col0;
@@ -366,7 +386,7 @@ __global__ void __launch_bounds__(TC3_THREADS, 1) joint_tc3_kernel(const __grid_
                 __syncwarp();
                 if (lane == 0) ptx::mbar_arrive(&acc_empty[buf]);
             }
-            if (MODE == 2 && has_slot) p.gm[rowbase + r] = ref;   // the row's reference (log2 domain), coalesced
+            if (MODE == 2 && has_slot) p.gm[rowbase + r] = ref;   // the row's final frame (log2 domain), coalesced
             if (rv && p.lse) {   // (lse == NULL: a backward-time recompute that only wants the kept activations)
                 const float lse2 = m2 + log2f(s);
                 p.lse[cell] = lse2 * LN2;

@@ -327,7 +327,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC3_THREADS, 1) join
             const bool rv = t < ti.Tn && u < ti.Un;
             const int lab = (rv && u < ti.Un - 1) ? p.labels[(size_t)ti.b * (p.maxU - 1) + u] : -1;
             const long long cell = ((long long)ti.b * p.maxT + t) * p.maxU + u;
-            float m2 = -CUDART_INF_F, s = 0.f, yb = 0.f, yl = 0.f, ref = 0.f;
+            float s = 0.f, yb = 0.f, yl = 0.f, ref = -CUDART_INF_F;
             const uint32_t lane_addr = acc0 + ((uint32_t)(warp * 32) << 16);
             for (int c = 0; c < NCH; ++c, ++g) {
                 const uint32_t buf = g % NBUF, use = g / NBUF;
@@ -358,15 +358,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC3_THREADS, 1) join
                             y[i] = fmaf(__uint_as_float(v[i]), LOG2E, __shfl_sync(0xffffffffu, bv, i));
                     }
                     {
-                        // The row sum is kept as (m2, s): sum = s * 2^m2.  m2 starts as the row's FIXED reference (the maximum of its
-                        // first 32 logits) and stays there unless a later logit exceeds ref + 100 (detected on the group's sum, no
-                        // running maximum is computed in the common path).  Both modes use the same arithmetic, hence identical costs
-                        // whether or not the numerators are kept.  MODE 2 stores the numerators 2^(y - ref) (bf16).
+                        // The row sum is kept as (ref, s): sum = s * 2^ref.  ref, the row's FRAME, starts as the maximum of its first
+                        // 32 logits and stays there unless a later group's sum against it reaches 2^64 (detected on the sum, no
+                        // running maximum is computed in the common path); the frame then moves up to that group's maximum.  Every
+                        // numerator 2^(y - ref) is thus below 2^64 and taken against the row's FINAL frame: MODE 2 stores them (bf16)
+                        // and rescales the ones already stored when the frame moves.  Both modes use the same arithmetic, hence
+                        // identical costs whether or not the numerators are kept.
                         if (col0 == 0) {
                             float gm = y[0];
 #pragma unroll
                             for (int i = 1; i < 32; ++i) gm = fmaxf(gm, y[i]);
-                            ref = gm; m2 = gm;
+                            ref = gm;
                         }
                         uint32_t o[16];
                         float accr = 0.f;
@@ -376,24 +378,27 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC3_THREADS, 1) join
                             accr += e0 + e1;
                             if (MODE == 2) o[i >> 1] = ptx::pack_bf16x2(e0, e1);
                         }
-                        if (accr < 1.0e30f) {            // every term below 2^100 (NaN / inf fail the test)
-                            s += (m2 == ref) ? accr : accr * ptx::ex2_approx(ref - m2);
+                        if (accr < 0x1p64f) {            // every term below 2^64 (NaN / inf fail the test)
+                            s += accr;
                         } else {
-                            // a logit about 2^100 above the reference (never seen outside adversarial inputs): the group's sum is
-                            // taken against its own maximum and the row switches to that frame; stored values are clamped at 2^100
+                            // a logit at least 59 bits above the frame (a confident row whose maximum lies beyond its first 32
+                            // columns): the group's numerators and sum are taken against its own maximum, the row switches to that
+                            // frame, and the numerators kept so far are brought into it
                             float gm = y[0];
 #pragma unroll
                             for (int i = 1; i < 32; ++i) gm = fmaxf(gm, y[i]);
-                            const float mn = fmaxf(m2, gm);
+                            const float mn = fmaxf(ref, gm);
                             float acc = 0.f;
 #pragma unroll
                             for (int i = 0; i < 32; i += 2) {
-                                acc += ptx::ex2_approx(y[i] - mn) + ptx::ex2_approx(y[i + 1] - mn);
-                                if (MODE == 2)
-                                    o[i >> 1] = ptx::pack_bf16x2(ptx::ex2_approx(fminf(y[i] - ref, 100.f)), ptx::ex2_approx(fminf(y[i + 1] - ref, 100.f)));
+                                const float e0 = ptx::ex2_approx(y[i] - mn), e1 = ptx::ex2_approx(y[i + 1] - mn);
+                                acc += e0 + e1;
+                                if (MODE == 2) o[i >> 1] = ptx::pack_bf16x2(e0, e1);
                             }
-                            s = s * ptx::ex2_approx(m2 - mn) + acc;
-                            m2 = mn;
+                            const float f = ptx::ex2_approx(ref - mn);
+                            if (MODE == 2 && has_slot) tc_rescale_kept(p.dl + (rowbase + r) * p.Vp, col0, f);
+                            s = s * f + acc;
+                            ref = mn;
                         }
                         if (MODE == 2 && has_slot) {
                             __nv_bfloat16* dst = p.dl + (rowbase + r) * p.Vp + col0;
@@ -428,9 +433,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC3_THREADS, 1) join
                 __syncwarp();
                 if (lane == 0) arrive_leader(&acc_empty[buf]);
             }
-            if (MODE == 2 && has_slot) p.gm[rowbase + r] = ref;   // the row's reference (log2 domain), coalesced
+            if (MODE == 2 && has_slot) p.gm[rowbase + r] = ref;   // the row's final frame (log2 domain), coalesced
             if (rv && p.lse) {   // (lse == NULL: a backward-time recompute that only wants the kept activations)
-                const float lse2 = m2 + log2f(s);
+                const float lse2 = ref + log2f(s);
                 p.lse[cell] = lse2 * LN2;
                 const long long k = sk_index(ti.b, t, u, p.maxU, p.SK);
                 p.lpb[k] = (yb - lse2) * LN2;

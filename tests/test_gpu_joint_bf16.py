@@ -135,8 +135,9 @@ def test_tc_edge_lattices(oracle, B, T, U, V, H, blank, keep):
 
 
 def test_large_magnitude_logits(oracle):
-    """Logits of magnitude ~40 (saturated softmax, numerators spanning the whole fp16 range below the running maximum):
-    costs and gradients stay finite and on the oracle."""
+    """Logits of magnitude ~40 (saturated softmax; the kept bf16 numerators span dozens of binades around the row's
+    frame, and a row's maximum lies up to ~28 bits above its first 32 logits -- far below the 2^64 frame switch, which
+    tests/test_gpu_joint_extreme_logits.py covers): costs and gradients stay finite and on the oracle."""
     k = synth(2, 24, 10, 128, 64, 9, ragged=True)
     k["W"] = (k["W"] * 12).astype(np.float32)
     k["b"] = (k["b"] * 30).astype(np.float32)
